@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's configurations.
 
-    python bench.py --gpus N --steps K --warmup W [--workload W] [--path P] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload W] [--path P] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 metric   : accepted RK steps/s x state elements, whole job (all ranks)
@@ -463,6 +463,33 @@ def timed(ctx, step_fn, steps, warmup):
     return dict(value=work / (ms * 1e-3), ms_per_step=ms / steps, launches=int(launches), wall=wall)
 
 
+DUMP_BYTES = 60 * 1000 * 1000       # --dump-outputs: data of all files together, under 64 MB with room for the headers
+
+
+def sample_outputs(arrays):
+    """Host copies of the arrays a caller of the timed path received from its last step (--dump-outputs).  `arrays` maps
+    a name to (tensor, batch axis or None).  Tensors with a batch axis keep the same rows: all of them when everything fits
+    in DUMP_BYTES, otherwise a sorted sample drawn with np.random.default_rng(0), so that runs with the same arguments
+    dump the same elements.  Tensors without a batch axis are kept whole."""
+    fixed = sum(t.numel() * t.element_size() for t, ax in arrays.values() if ax is None)
+    batched = [(t, ax) for t, ax in arrays.values() if ax is not None]
+    idx = None
+    if batched:
+        n = batched[0][0].shape[batched[0][1]]
+        assert all(t.shape[ax] == n for t, ax in batched)
+        per_row = sum(t.numel() // n * t.element_size() for t, ax in batched)
+        rows = min(n, (DUMP_BYTES - fixed) // per_row)
+        if rows < n:
+            idx = np.sort(np.random.default_rng(0).choice(n, size=rows, replace=False))
+    out = {}
+    for name, (t, ax) in arrays.items():
+        t = t.detach()
+        if ax is not None and idx is not None:
+            t = t.index_select(ax, torch.from_numpy(idx).to(t.device))
+        out[name] = t.cpu().numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32, copy=False)
+    return out
+
+
 def make_solver(ctx, w, path, host_output=None):
     """Closures for one workload / path: solve(y_dev) -> solution, plus bookkeeping of accepted steps."""
     import tfdiffeq_b200 as tfd
@@ -488,7 +515,7 @@ def graph_launches(stats, n_k_minus_1_plus_2):
     return max(stats["n_accepted"] + stats["n_rejected"] - 2, 0) * n_k_minus_1_plus_2
 
 
-def run_odeint_workload(ctx, w, path, steps, warmup, want_e2e=True):
+def run_odeint_workload(ctx, w, path, steps, warmup, want_e2e=True, keep_output=False):
     import tfdiffeq_b200 as tfd
     solve, _ = make_solver(ctx, w, path)
     y0_host = torch.from_numpy(np.ascontiguousarray(w.y0(ctx.rank))).pin_memory()
@@ -496,13 +523,18 @@ def run_odeint_workload(ctx, w, path, steps, warmup, want_e2e=True):
     nk = {"dopri5": 8, "dopri8": 15, "rk4": 0}.get(w.method, 0)
     n_el = w.elements()
     stats_box = {}
+    last = {}
 
     def step_dev():
-        solve(y0_dev)
+        sol = solve(y0_dev)
+        if keep_output:
+            last["solution"] = sol
         s = tfd.last_stats
         stats_box.update(s)
         return float(s["n_accepted"]) * n_el, graph_launches(s, nk)
     res = timed(ctx, step_dev, steps, max(warmup, 3))
+    if keep_output:
+        res["outputs"] = sample_outputs({"solution": (last.pop("solution"), 1)})
     res["n_acc"], res["n_rej"] = stats_box.get("n_accepted"), stats_box.get("n_rejected")
     res["fused_rhs"] = bool(stats_box.get("fused_rhs"))
     if want_e2e:
@@ -588,7 +620,7 @@ def parity_odeint(ctx, w, path):
 
 
 # ---- config 4: forward + adjoint ---------------------------------------------------------------------------------------
-def run_cfg4(ctx, w, path, steps, warmup):
+def run_cfg4(ctx, w, path, steps, warmup, keep_output=False):
     import tfdiffeq_b200 as tfd
     from tfdiffeq_b200 import adjoint as adj
     torch.manual_seed(0)
@@ -618,12 +650,19 @@ def run_cfg4(ctx, w, path, steps, warmup):
             gp_host.copy_(torch.cat([p.grad.reshape(-1) for p in m.parameters()]), non_blocking=True)
             box["loss"] = float(loss)                               # D2H read of the step's result
             torch.cuda.synchronize(ctx.dev)
+        elif keep_output:
+            box["outputs"] = (out, x, [p.grad for p in m.parameters()])
         fwd, bwd = adj.last_stats["forward"], adj.last_stats["backward"]
         box.update(fwd_acc=fwd["n_accepted"], fwd_rej=fwd["n_rejected"], bwd_acc=sum(b["n_accepted"] for b in bwd),
                    bwd_rej=sum(b["n_rejected"] for b in bwd), nfe=m.nfe)
         return float(fwd["n_accepted"]) * n_el + float(sum(b["n_accepted"] for b in bwd)) * n_aug, 0
     x_dev = x_host.to(ctx.dev)
     res = timed(ctx, lambda: step(False), steps, warmup)
+    if keep_output:
+        out, x, grads = box.pop("outputs")
+        res["outputs"] = sample_outputs({"solution": (out, 1), "input_grad": (x.grad, 0),
+                                         "param_grad": (torch.cat([g.reshape(-1) for g in grads]), None)})
+        del out, x, grads
     e = timed(ctx, lambda: step(True), max(1, min(steps, 3)), 1)
     res["e2e"] = {"value": e["value"], "unit": UNIT, "ms_per_step": e["ms_per_step"],
                   "h2d_bytes_per_step": int(x_host.numel() * 4), "d2h_bytes_per_step": int(gx_host.numel() * 4 + n_par * 4 + 4)}
@@ -837,13 +876,13 @@ def tensor_core_block(ctx):
     return out
 
 
-def run_workload(ctx, name, path, steps, warmup, want_parity=True):
+def run_workload(ctx, name, path, steps, warmup, want_parity=True, keep_output=False):
     w = WORKLOADS[name]
     path = path or w.paths[0]
     if name == "cfg4":
-        res = run_cfg4(ctx, w, path, steps, warmup)
+        res = run_cfg4(ctx, w, path, steps, warmup, keep_output)
     else:
-        res = run_odeint_workload(ctx, w, path, steps, warmup)
+        res = run_odeint_workload(ctx, w, path, steps, warmup, keep_output=keep_output)
         if want_parity:
             res["parity"] = parity_odeint(ctx, w, path)
     res["path"] = path
@@ -862,7 +901,14 @@ def run_ours(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    main = run_workload(ctx, primary_name, primary_path, args.steps, max(args.warmup, 3))
+    main = run_workload(ctx, primary_name, primary_path, args.steps, max(args.warmup, 3),
+                        keep_output=args.dump_outputs is not None)
+    outputs = main.pop("outputs", {})
+    if rank == 0 and outputs:                                      # at N > 1: rank 0's shard
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+    del outputs
     others_paths = {}
     if primary_name != "cfg4":
         for p in w.paths:
@@ -944,7 +990,14 @@ def main():
     ap.add_argument("--path", default=None, help="which public-API path of the workload is the primary (timed) one")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="primary workload only: skip other_workloads / tensor_core_func / cpu_baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the primary path returned in its last timed step to DIR/<name>.npy (float32 / float64, "
+                         "a seeded sample of the batch rows, under 64 MB in all), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -5,6 +5,8 @@ For every case of tests/cases.py the reference's own ``odeint`` (tfdiffeq/odeint
 oracle/tf_shim.py because TensorFlow is not installable here) is run on torch-CPU tensors, and the
 solution (time axis subsampled by ``keep``), the accepted / rejected / NFE counts and the dt trace are
 stored.  The fixtures travel to the GPU box; the reference does not.
+The reference's literal Adams tables go to tests/golden/adams_tables.npz (``python oracle/make_golden.py adams_tables``
+writes only those).
 """
 import os
 import signal
@@ -92,10 +94,22 @@ def run_case(c):
     return res
 
 
+def adams_tables():
+    """The reference's literal Adams-Bashforth / Adams-Moulton tables and divisors (tfdiffeq/fixed_adams.py:8-145), one
+    comma-separated row of decimal integers per order (index 0 is empty): the high orders do not fit in int64."""
+    fa = ref_loader.load().fixed_adams
+    row = lambda r: ",".join(str(int(x)) for x in r)                     # noqa: E731
+    return dict(bashforth=np.array([row(r) for r in fa._BASHFORTH_COEFFICIENTS]),
+                moulton=np.array([row(r) for r in fa._MOULTON_COEFFICIENTS]),
+                divisor=np.array(["" if d is None else str(int(d)) for d in fa._DIVISOR]))
+
+
 def main():
     outdir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(outdir, exist_ok=True)
     only = sys.argv[1:]
+    if not only or "adams_tables" in only:
+        np.savez_compressed(os.path.join(outdir, "adams_tables.npz"), **adams_tables())
     for c in CASES:
         if only and c["name"] not in only:
             continue

@@ -158,10 +158,10 @@ def test_product_never_imports_the_oracle():
             assert "np_ref" not in src and "import oracle" not in src and "from oracle" not in src, fn
 
 
-def test_adams_weights_are_exact_and_match_the_oracle():
+def test_adams_weights_are_exact_and_match_the_oracle(golden_dir):
     """The product regenerates the Adams-Bashforth / Adams-Moulton tables (tfdiffeq/fixed_adams.py:7-160) from their
-    definition; the oracle does so independently and was compared entry by entry with the reference's literal tables
-    when the golden vectors were made (oracle/make_golden.py)."""
+    definition; the oracle does so independently.  Both are compared entry by entry with the reference's literal tables,
+    stored by oracle/make_golden.py in tests/golden/adams_tables.npz as decimal strings."""
     from fractions import Fraction
     from tfdiffeq_b200.multistep import adams_weights
     for k in range(1, 21):
@@ -172,14 +172,11 @@ def test_adams_weights_are_exact_and_match_the_oracle():
     assert adams_weights(4, False) == ([55, -59, 37, -9], 24)
     assert adams_weights(4, True) == ([9, 19, -5, 1], 24)
     assert adams_weights(5, True) == ([251, 646, -264, 106, -19], 720)
-    ref = os.path.join(os.sep, "root", "reference", "tfdiffeq", "fixed_adams.py")
-    if os.path.exists(ref):                                            # build container only
-        ns = {}
-        src = open(ref).read()
-        exec(src[src.index("_BASHFORTH_COEFFICIENTS"):src.index("_MIN_ORDER")], ns)   # the three literal tables, nothing else
-        for k in range(2, 21):
-            assert adams_weights(k, False) == (ns["_BASHFORTH_COEFFICIENTS"][k], ns["_DIVISOR"][k])
-            assert adams_weights(k, True) == (ns["_MOULTON_COEFFICIENTS"][k], ns["_DIVISOR"][k])
+    g = np.load(os.path.join(golden_dir, "adams_tables.npz"))
+    ints = lambda s: [int(x) for x in str(s).split(",")]                # noqa: E731
+    for k in range(2, 21):
+        assert adams_weights(k, False) == (ints(g["bashforth"][k]), int(g["divisor"][k]))
+        assert adams_weights(k, True) == (ints(g["moulton"][k]), int(g["divisor"][k]))
 
 
 def test_multistep_host_controller_matches_the_oracle():
