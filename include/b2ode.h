@@ -202,13 +202,17 @@ int b2ode_comm_set_replicated(b2ode_solver *s, unsigned segment_mask);
                                        [W1 (2 x H) | b1 (H) | W2 (H x 2) | b2 (2)] in the state dtype   examples/ode_demo.py:115-129 */
 
 #define B2ODE_RHS_KEPLER 3         /* (B, 4 m): m two-body orbits [x, y, vx, vy] per row; no params   tests/DETEST/detest.py:263-283 */
+#define B2ODE_RHS_LINEAR 4         /* (B, D): y @ A (+ b), k[r, c] = sum_d y[r, d] A[d, c]; params {D, has_bias}, 1 <= D <= 128;
+                                      data = A row-major D x D in the state dtype, then b (D values) iff has_bias.  Stage
+                                      kernels only (b2ode_rhs_eval / b2ode_rk_stage_rhs, fp64 GEMM on DMMA): b2ode_fused_capacity
+                                      returns 0 and the persistent / fixed-grid solves reject it   tests/problems.py:43-68 */
 
 /* A built-in right-hand side as the kernels see it. */
 typedef struct b2ode_rhs_desc {
     int32_t kind;                       /* B2ODE_RHS_*                                                   */
     int32_t n_params;
     double params[8];
-    const void *data;                   /* staged weights (B2ODE_RHS_CUBIC_MLP), else NULL               */
+    const void *data;                   /* staged weights (B2ODE_RHS_CUBIC_MLP, B2ODE_RHS_LINEAR), else NULL */
     double time_sign;                   /* -1: the reversed system of tfdiffeq/misc.py:318-321           */
 } b2ode_rhs_desc;
 
@@ -336,6 +340,8 @@ int b2ode_mlp3(const void *x, const void *const *k, const double *coef, int nk, 
 
 /* ---- measurement hooks (bench.py) --------------------------------------------------------------------- */
 unsigned long long b2ode_launch_count(void);            /* kernels launched by this library so far          */
+/* families: 0 stage 0, 1 stage, 2 finalize, 3 dense output, 4 initial step, 5 fixed grid, 6 persistent solve,
+ * 7 linear stage GEMM (B2ODE_RHS_LINEAR's stage / evaluation kernel) */
 int b2ode_timing_enable(unsigned family_mask);          /* CUDA-event timing per kernel family; 0 = off     */
 int b2ode_timing_read(int family, double *total_ms, int *count);
 

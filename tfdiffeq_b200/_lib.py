@@ -12,8 +12,9 @@ MAXPEERS = 8
 F32, F64 = 0, 1
 ST_UNDERFLOW, ST_NONFINITE, ST_MAXSTEPS = 1, 2, 4
 CTRL_REFERENCE, CTRL_TSIT5 = 0, 1
-FAM_STAGE0, FAM_STAGE, FAM_FINALIZE, FAM_EMIT, FAM_INIT, FAM_FIXED, FAM_FUSED = range(7)
-RHS_LORENZ, RHS_LOTKA_VOLTERRA, RHS_CUBIC_MLP, RHS_KEPLER = 0, 1, 2, 3
+FAM_STAGE0, FAM_STAGE, FAM_FINALIZE, FAM_EMIT, FAM_INIT, FAM_FIXED, FAM_FUSED, FAM_STAGE_GEMM = range(8)
+RHS_LORENZ, RHS_LOTKA_VOLTERRA, RHS_CUBIC_MLP, RHS_KEPLER, RHS_LINEAR = 0, 1, 2, 3, 4
+LINEAR_MAX_DIM = 128      # largest D of RHS_LINEAR (A stays in shared memory: 128 x 128 fp64 = 128 KB)
 OP_EULER, OP_HALF_STEP, OP_HEUN_FINAL, OP_RK4_S2, OP_RK4_S3, OP_RK4_S4, OP_RK4_FINAL, OP_LERP = range(8)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))

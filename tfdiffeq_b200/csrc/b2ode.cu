@@ -1063,7 +1063,9 @@ extern "C" int b2ode_comm_set_replicated(b2ode_solver *s, unsigned segment_mask)
 static unsigned long long g_launches = 0;
 void b2_count_launch(void) { ++g_launches; }
 
-enum { B2_FAM_STAGE0 = 0, B2_FAM_STAGE = 1, B2_FAM_FINALIZE = 2, B2_FAM_EMIT = 3, B2_FAM_INIT = 4, B2_FAM_FIXED = 5, B2_FAM_FUSED = 6, B2_NFAM = 7 };
+enum { B2_FAM_STAGE0 = 0, B2_FAM_STAGE = 1, B2_FAM_FINALIZE = 2, B2_FAM_EMIT = 3, B2_FAM_INIT = 4, B2_FAM_FIXED = 5, B2_FAM_FUSED = 6,
+       B2_FAM_STAGE_GEMM = 7, B2_NFAM = 8 };
+static_assert(B2_FAM_STAGE_GEMM == kFamStageGemm, "linear stage kernel timing family");
 constexpr int kMaxTimed = 2048;   // event pairs per family
 
 struct Timing {
@@ -1110,7 +1112,8 @@ void b2_timing_end(int fam, int slot, cudaStream_t st) {
 }
 
 // Enable CUDA-event timing of the kernel families in `family_mask` (bit f = family f: 0 stage0, 1 stage,
-// 2 finalize, 3 dense output, 4 initial step, 5 fixed grid, 6 fused persistent solve); 0 disables.  Resets the counters.
+// 2 finalize, 3 dense output, 4 initial step, 5 fixed grid, 6 fused persistent solve, 7 linear stage GEMM); 0 disables.
+// Resets the counters.
 extern "C" int b2ode_timing_enable(unsigned family_mask) {
     if (!g_timing) {
         g_timing = new (std::nothrow) Timing();
@@ -1342,12 +1345,13 @@ extern "C" int b2ode_rk_stage(b2ode_solver *s, int i, const void *const *k_new) 
 }
 
 // ---- stage kernels with a built-in right-hand side ------------------------------------------------------------------
-static int rhs_row_dim(int kind) {
-    switch (kind) {
+static int rhs_row_dim(const b2ode_rhs_desc *r) {
+    switch (r->kind) {
         case B2ODE_RHS_LORENZ: return 3;
         case B2ODE_RHS_LOTKA_VOLTERRA:
         case B2ODE_RHS_CUBIC_MLP: return 2;
         case B2ODE_RHS_KEPLER: return 4;
+        case B2ODE_RHS_LINEAR: return r->n_params >= 1 ? (int)r->params[0] : -1;
     }
     return -1;
 }
@@ -1367,9 +1371,32 @@ static int launch_stage_rhs_t(const StageRhsParams<NK> &p, int sm_count, cudaStr
     return launch(k_rk_stage_rhs<T, RHS, NK>, grid, st, p, B2_FAM_STAGE);
 }
 
+// B2ODE_RHS_LINEAR: the stage combine feeds a DMMA GEMM in b2ode_linear.cu (its own kernel, timing family 7)
+template <typename T, int NK>
+static int launch_stage_linear(const StageRhsParams<NK> &p, int sm_count, cudaStream_t st) {
+    LinearStageArgs a;
+    memset(&a, 0, sizeof(a));
+    a.st = p.st;
+    a.y0 = p.y0;
+    for (int j = 0; j < NK; ++j) {
+        a.k[j] = p.k[j];
+        a.coef[j] = p.coef[j];
+    }
+    a.nk = NK;
+    a.ystage = p.ystage;
+    a.k_out = p.k_out;
+    a.rows = p.rows;
+    a.D = (int)p.rhs[0];
+    a.has_bias = p.rhs[1] != 0.0;
+    a.data = p.rhs_data;
+    a.time_sign = p.time_sign;
+    return b2_launch_stage_linear(std::is_same<T, double>::value ? B2ODE_F64 : B2ODE_F32, a, sm_count, st);
+}
+
 template <typename T, int NK>
 static int launch_stage_rhs_k(int kind, const StageRhsParams<NK> &p, int sm_count, cudaStream_t st) {
     switch (kind) {
+        case B2ODE_RHS_LINEAR: return launch_stage_linear<T, NK>(p, sm_count, st);
         case B2ODE_RHS_LORENZ: return launch_stage_rhs_t<T, RhsLorenz<T>, NK>(p, sm_count, st);
         case B2ODE_RHS_LOTKA_VOLTERRA: return launch_stage_rhs_t<T, RhsLotkaVolterra<T>, NK>(p, sm_count, st);
         case B2ODE_RHS_CUBIC_MLP: return launch_stage_rhs_t<T, RhsCubicMLP<T>, NK>(p, sm_count, st);
@@ -1387,9 +1414,15 @@ static void fill_rhs(StageRhsParams<NK> *p, const b2ode_rhs_desc *r) {
 
 static int check_rhs(const b2ode_rhs_desc *r, long long seg_len, long long *rows) {
     if (!r) return b2_fail(B2ODE_EINVAL, "null right-hand side");
-    const int D = rhs_row_dim(r->kind);
-    if (D < 0) return b2_fail(B2ODE_EINVAL, "unknown built-in right-hand side %d", r->kind);
     if (r->n_params < 0 || r->n_params > 8) return b2_fail(B2ODE_EINVAL, "bad rhs params");
+    if (r->kind == B2ODE_RHS_LINEAR) {
+        const double d = r->n_params >= 1 ? r->params[0] : 0.0;
+        if (!(d >= 1.0 && d <= (double)kLinearMaxD) || d != (double)(int)d)
+            return b2_fail(B2ODE_EINVAL, "linear right-hand side needs params {D, has_bias} with 1 <= D <= %d", kLinearMaxD);
+        if (!r->data) return b2_fail(B2ODE_EINVAL, "linear right-hand side needs its matrix (rhs data)");
+    }
+    const int D = rhs_row_dim(r);
+    if (D < 0) return b2_fail(B2ODE_EINVAL, "unknown built-in right-hand side %d", r->kind);
     if (seg_len % D != 0) return b2_fail(B2ODE_EINVAL, "state length %lld is not a multiple of the row size %d", seg_len, D);
     if (r->kind == B2ODE_RHS_CUBIC_MLP && (!r->data || r->n_params < 2 || r->params[0] < 1 || r->params[0] > 128))
         return b2_fail(B2ODE_EINVAL, "cubic-MLP right-hand side needs {H <= 128, cube} and its weights");

@@ -1041,6 +1041,7 @@ static int fused_dispatch_rhs(const FusedParams &p, int rhs_kind, int n_k, long 
 // side: the host asks BEFORE launching, so that the shards of a shared-step group can agree on one path.  < 0: error.
 extern "C" int64_t b2ode_fused_capacity(const b2ode_adaptive_desc *desc, int rhs_kind) {
     if (!desc) return b2_fail(B2ODE_EINVAL, "null argument");
+    if (rhs_kind == B2ODE_RHS_LINEAR) return 0;     // a row of up to 128 values does not fit one thread's registers
     FusedParams p;
     memset(&p, 0, sizeof(p));
     long long cap = 0;
@@ -1074,6 +1075,7 @@ extern "C" int b2ode_fused_solve(const b2ode_adaptive_desc *desc, const b2ode_fu
     if (!desc || !f) return b2_fail(B2ODE_EINVAL, "null argument");
     if (!f->y0 || !f->out || !f->t_out || !f->state || !f->workspace) return b2_fail(B2ODE_EINVAL, "null buffer");
     const int rhs_kind = f->rhs_kind;
+    if (rhs_kind == B2ODE_RHS_LINEAR) return b2_fail(B2ODE_EINVAL, "the linear right-hand side has no persistent kernel");
     const int D = rhs_dim(rhs_kind);
     if (D < 0) return b2_fail(B2ODE_EINVAL, "unknown built-in right-hand side %d", rhs_kind);
     if (desc->nseg != 1 || desc->seg_len[0] % D != 0) return b2_fail(B2ODE_EINVAL, "state must be one (B, %d) tensor", D);
@@ -1285,6 +1287,7 @@ extern "C" int b2ode_fused_fixed_solve(int dtype, int method, int rhs_kind, cons
     if (!y0 || !out || n_traj < 1 || n_out < 1 || n_steps < 0) return b2_fail(B2ODE_EINVAL, "bad arguments");
     if (n_steps > 0 && (!times || !dts || !j0 || !ends || !s1 || !s2)) return b2_fail(B2ODE_EINVAL, "null grid array");
     if (method < 0 || method > 3) return b2_fail(B2ODE_EINVAL, "method must be 0..3");
+    if (rhs_kind == B2ODE_RHS_LINEAR) return b2_fail(B2ODE_EINVAL, "the linear right-hand side has no one-launch fixed-grid kernel");
     if (rhs_dim(rhs_kind) < 0) return b2_fail(B2ODE_EINVAL, "unknown built-in right-hand side %d", rhs_kind);
     if (n_rhs_params < 0 || n_rhs_params > 8 || (n_rhs_params && !rhs_params)) return b2_fail(B2ODE_EINVAL, "bad rhs params");
     const int rc = rhs_check(rhs_kind, rhs_params, n_rhs_params, rhs_data);

@@ -62,6 +62,25 @@ struct RhsCubicMLP {
 };
 
 
+// B2ODE_RHS_LINEAR (rhs.py's LinearSystem): k = s * (y @ A + b) on rows of D <= 128, with the stage combine fused in front of
+// the GEMM (b2ode_linear.cu).  Rows do not fit one thread's registers, so this kind has its own kernel rather than an eval().
+constexpr int kLinearMaxD = 128;
+constexpr int kFamStageGemm = 7;   // B2_FAM_STAGE_GEMM: timing family of the linear stage kernel (b2ode.cu)
+struct LinearStageArgs {
+    const b2ode_state *st;
+    const void *y0;
+    const void *k[B2ODE_MAXK];
+    double coef[B2ODE_MAXK];
+    int nk;                      // stage terms, 0 = plain evaluation of y0
+    void *ystage;                // optional: also store the stage input (the last stage's input is y1)
+    void *k_out;
+    long long rows;
+    int D, has_bias;
+    const void *data;            // A (D x D row-major), then b (D) if has_bias; state dtype
+    double time_sign;
+};
+int b2_launch_stage_linear(int dtype, const LinearStageArgs &a, int sm_count, cudaStream_t st);
+
 // DETEST class D (tests/DETEST/detest.py:263-283): a two-body orbit, state [x, y, vx, vy] per row; BASELINE config 5 stacks 32
 // of them per batch row (dim 128), i.e. the (B, 128) state is (32 B) rows of 4.  r^3 = (x^2 + y^2)^1.5 like the torch module.
 template <typename T>

@@ -19,6 +19,7 @@ from . import _lib
 class BuiltinRHS(nn.Module):
     kind = None      # B2ODE_RHS_* code
     dim = None       # size of the last state axis
+    persistent = True   # has a one-launch form (persistent adaptive kernel, fixed-grid kernel); else stage kernels only
 
     def rhs_params(self):
         raise NotImplementedError
@@ -103,6 +104,52 @@ class CubicMLP(BuiltinRHS):
     def forward(self, t, y):
         u = y ** 3 if self.cube else y
         return torch.tanh(u @ self.W1 + self.b1) @ self.W2 + self.b2
+
+
+class LinearSystem(BuiltinRHS):
+    """The linear system ``y' = y @ A (+ b)`` on a ``(..., D)`` state (the reference's ``LinearODE`` fixture,
+    tests/problems.py:43-68, and the north-star ``BatchedLinear`` workload).  ``A`` (D x D) and ``b`` (D) are
+    ``nn.Parameter`` s and ``forward`` is plain torch, so the module trains and runs anywhere.
+
+    Note the side: unlike ``nn.Linear`` (``x @ W.T``) the state multiplies ``A`` from the LEFT, ``k[r, c] = sum_d
+    y[r, d] A[d, c]`` -- as in ``BatchedLinear`` and ode_demo.py's ``y**3 @ A``.  A column-vector system ``x' = M x`` is
+    ``LinearSystem(M.T)``.
+
+    With an adaptive Runge-Kutta method on a CUDA state and ``D <= 128`` the solver runs every stage as ONE launch
+    (``b2ode_rk_stage_rhs``): the stage combine forms the stage input tile by tile in shared memory and feeds it straight
+    into an fp64 GEMM on the DMMA tensor cores with ``A`` resident in shared memory (fp32 states: fp32 FMAs), so the stage
+    input never round-trips HBM and ``forward`` is never called.  There is no persistent one-kernel form (a row of up to 128
+    values does not fit one thread's registers).  Fixed-grid and multistep methods, ``D > 128`` (with a warning) and
+    ``options={'fused_rhs': False}`` call ``forward``."""
+    kind = _lib.RHS_LINEAR
+    persistent = False
+
+    def __init__(self, A, b=None):
+        super(LinearSystem, self).__init__()
+        A = torch.as_tensor(A)
+        if A.dim() != 2 or A.shape[0] != A.shape[1] or A.shape[0] < 1:
+            raise ValueError("A must be a square (D, D) matrix")
+        self.dim = int(A.shape[0])
+        self.A = nn.Parameter(A.detach().clone())
+        if b is not None:
+            b = torch.as_tensor(b, dtype=A.dtype, device=A.device)
+            if b.shape != (self.dim,):
+                raise ValueError("b must have shape (D,)")
+            self.b = nn.Parameter(b.detach().clone())
+        else:
+            self.b = None
+
+    def rhs_params(self):
+        return [float(self.dim), 0.0 if self.b is None else 1.0]
+
+    def rhs_data(self, dtype, device):
+        with torch.no_grad():
+            parts = [self.A.reshape(-1)] + ([] if self.b is None else [self.b.reshape(-1)])
+            return torch.cat([p.to(device=device, dtype=dtype) for p in parts]).contiguous()
+
+    def forward(self, t, y):
+        k = y @ self.A
+        return k if self.b is None else k + self.b
 
 
 _ACT = {None: 0, "none": 0, "relu": 1, "tanh": 2, "softplus": 3}

@@ -180,7 +180,8 @@ class AdaptiveStepsizeODESolver(object):
         self.cuda_graph = bool(unused_kwargs.pop("cuda_graph", False))
         # extension: a built-in right-hand side (tfdiffeq_b200/rhs.py) runs in one persistent kernel unless disabled
         # (True: persistent kernel when the batch fits, else the stage kernels with the right-hand side fused in; 'stages':
-        # always the latter; False: call func like any other callable)
+        # always the latter; False: call func like any other callable).  rhs.LinearSystem has no persistent kernel:
+        # True and 'stages' both take its stage kernels
         fr = unused_kwargs.pop("fused_rhs", True)
         self.fused_rhs = fr if fr == "stages" else bool(fr)
         # extension: a page-locked host tensor of the solution's shape.  The solution is delivered THERE (and returned as
@@ -270,7 +271,8 @@ class AdaptiveStepsizeODESolver(object):
         from .rhs import BuiltinRHS
         base = getattr(self.func, "_b2ode_base", None)
         tab = self.tableau
-        if not isinstance(base, BuiltinRHS) or seg.nseg != 1 or tab.c_mid is None or tab.n_k not in (2, 4, 7, 14):
+        if (not isinstance(base, BuiltinRHS) or not base.persistent or seg.nseg != 1 or tab.c_mid is None
+                or tab.n_k not in (2, 4, 7, 14)):
             return None
         shape = seg.shapes[0]
         if len(shape) < 1 or shape[-1] % base.dim != 0 or seg.lens[0] == 0:
@@ -409,6 +411,12 @@ class AdaptiveStepsizeODESolver(object):
             brhs = getattr(self.func, "_b2ode_base", None)
             if not (self.fused_rhs and isinstance(brhs, BuiltinRHS) and seg.nseg == 1 and len(seg.shapes[0]) >= 1
                     and seg.shapes[0][-1] % brhs.dim == 0 and seg.lens[0] > 0):
+                brhs = None
+            elif brhs.kind == _lib.RHS_LINEAR and (seg.shapes[0][-1] != brhs.dim or brhs.dim > _lib.LINEAR_MAX_DIM):
+                if brhs.dim > _lib.LINEAR_MAX_DIM:
+                    import warnings
+                    warnings.warn("tfdiffeq_b200: LinearSystem of dimension %d exceeds the stage kernel's limit of %d (A must "
+                                  "fit in shared memory); calling its forward" % (brhs.dim, _lib.LINEAR_MAX_DIM), RuntimeWarning)
                 brhs = None
             if brhs is not None:
                 rd = _lib.RhsDesc()
@@ -738,8 +746,8 @@ class FixedGridODESolver(object):
         # ---- built-in right-hand side: the whole grid in one launch (b2ode_fused_fixed_solve) -----------------------
         from .rhs import BuiltinRHS
         base = getattr(self.func, "_b2ode_base", None)
-        if (self.fused_rhs and isinstance(base, BuiltinRHS) and seg.nseg == 1 and len(seg.shapes[0]) >= 1
-                and seg.shapes[0][-1] % base.dim == 0 and seg.lens[0] > 0):
+        if (self.fused_rhs and isinstance(base, BuiltinRHS) and base.persistent and seg.nseg == 1
+                and len(seg.shapes[0]) >= 1 and seg.shapes[0][-1] % base.dim == 0 and seg.lens[0] > 0):
             n_traj = seg.lens[0] // base.dim
             j0 = np.zeros(n_steps + 1, dtype=np.int32)
             ends = np.zeros(max(n_steps, 1), dtype=np.uint8)
